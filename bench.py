@@ -3,7 +3,7 @@
 batches of the BASELINE.json configurations.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
-                    [--config c2|c3|c4|c5|c2small|c3small|c4small] [--dist uniform|zipf]
+                    [--config c2|c3|c4|c5|c2small|c3small|c4small] [--dist uniform|zipf] [--dump-outputs DIR]
 
 Default = BASELINE.json configs[1] (C2: DeepFM, 26 tables x 1M rows, emb_dim 32, batch 65536 per GPU); c3 =
 xDeepFM / CIN (128,128), emb_dim 16, batch 32768; c4 = DIN, 100k items, T=50, emb_dim 64, batch 8192; c5 =
@@ -15,8 +15,10 @@ already resident in HBM; `e2e` = the same step through the public API (`Model.fi
 pinned-H2D copy of the inputs and the D2H read of the loss; `roofline` = the dominant kernel group against the
 measured peaks in MEASURED_PEAKS.json (ALGORITHMIC bytes / flops of SURVEY.md section 8(d) over CUDA-event
 time); `cpu_baseline` = the CPU oracle (torch-CPU restatement of the reference math) on a bounded sample.
-`--impl reference` times the reference's CPU path: real TensorFlow + /root/reference's deepctr if importable
-(it is not in this image), else the oracle port - on the SAME config, steps and warm-up.
+`--impl reference` times the reference's CPU path: real TensorFlow + the reference's deepctr under baseline/_ref if
+importable, else the oracle port - on the SAME config, steps and warm-up.
+`--dump-outputs DIR` writes what the last timed step left for its caller (see dump_outputs) as DIR/<name>.npy; the
+inputs and initial weights are seeded, so two builds run with the same arguments can be compared file by file.
 """
 import argparse
 import json
@@ -304,6 +306,35 @@ def op_alone_us(make, reps=5):
     return timed_alone(g.replay, reps, flush)
 
 
+DUMP_ROWS = 2048          # rows kept per embedding table by --dump-outputs
+DUMP_LIMIT = 64 << 20     # bytes
+
+
+def dump_outputs(out_dir, loss_sum, model):
+    """Write, as float32 .npy files, what a training step leaves for its caller: the summed batch loss
+    train_step returned (loss_sum.npy) and every weight it trained (<weight name with '/' as '.'>.npy).
+    Tables with more than DUMP_ROWS rows are cut to a fixed, seeded sample of DUMP_ROWS rows (the same
+    rows in every run) so that the files stay below DUMP_LIMIT bytes.  Under several GPUs these are
+    rank 0's weights, i.e. its shard of each row-sharded table."""
+    import torch
+    arrays = {"loss_sum": loss_sum.detach().reshape(-1).cpu().numpy()}
+    rng = np.random.RandomState(0)
+    for w in model.weights:
+        t = w.data
+        if t is None:
+            continue
+        if t.dim() >= 1 and t.shape[0] > DUMP_ROWS:
+            rows = np.sort(rng.choice(t.shape[0], DUMP_ROWS, replace=False))
+            t = t.index_select(0, torch.from_numpy(rows).to(t.device))
+        arrays[w.name.replace("/", ".")] = t.detach().cpu().numpy().astype(np.float32)
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_LIMIT:
+        raise SystemExit("bench.py: --dump-outputs would write %d bytes (limit %d)" % (total, DUMP_LIMIT))
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 # ================================================================================================
 # CPU arm: the reference math on host cores
 # ================================================================================================
@@ -441,16 +472,16 @@ def run_cpu(cfg, steps, warmup, batch, dist):
 
 
 def run_tensorflow(cfg, steps, warmup, batch, dist):
-    """The real thing, when it can be imported: TensorFlow + the UNMODIFIED reference package (baseline/_ref or
-    /root/reference) - model.train_on_batch on the same synthetic batches, SGD, l2 = 0, all host cores.
+    """The real thing, when it can be imported: TensorFlow + the UNMODIFIED reference package (baseline/_ref)
+    - model.train_on_batch on the same synthetic batches, SGD, l2 = 0, all host cores.
     Returns None when TensorFlow / the reference cannot be imported (this image: always)."""
     try:
         import tensorflow as tf                                   # noqa: F401
     except Exception:
         return None
-    for p in (os.path.join(ROOT, "baseline", "_ref"), "/root/reference"):
-        if os.path.isdir(os.path.join(p, "deepctr")) and p not in sys.path:
-            sys.path.insert(0, p)
+    p = os.path.join(ROOT, "baseline", "_ref")
+    if os.path.isdir(os.path.join(p, "deepctr")) and p not in sys.path:
+        sys.path.insert(0, p)
     try:
         from deepctr import models as RM, feature_column as RFC
     except Exception:
@@ -490,7 +521,12 @@ def main():
     ap.add_argument("--cpu-sample-batch", type=int, default=8192)
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-e2e", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's outputs as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b2ctr":
+        ap.error("--dump-outputs applies to --impl b2ctr")
     world = int(os.environ.get("WORLD_SIZE", "1"))
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
@@ -542,6 +578,11 @@ def main():
         precision = "bf16x3"
     ops.set_gemm_precision(precision)
     model = build_model(cfg, act=args.din_act)
+    # the builders leave the output Dense's initializer unseeded, as the reference does; seed it so that every
+    # run starts from the same weights
+    for i, w in enumerate(model.weights):
+        if getattr(w.initializer, "seed", 0) is None:
+            w.initializer.seed = i
     model.compile(SGD(LR), "binary_crossentropy", embedding_update="sparse")
     host = synth_batches(cfg, N_BATCHES, rank, args.dist)
     dev = torch.device("cuda", local_rank)
@@ -571,13 +612,15 @@ def main():
     barrier()
     e0.record()
     for i in range(args.steps):
-        model.train_step(*dev_batches[(warmup_done + i) % N_BATCHES])
+        loss_sum = model.train_step(*dev_batches[(warmup_done + i) % N_BATCHES])
     e1.record()
     barrier()
     launches = L.launch_count() + model.replayed_launches
     graph_replays = args.steps if model._step_graphs else 0
     sampler.stop_flag = True
     ms = e0.elapsed_time(e1)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, loss_sum, model)
     # per-kernel durations: the same K steps once more, launched eagerly with a CUDA-event pair around every
     # kernel group (the timed region above replays graphs, which cannot carry per-kernel events)
     K.PROFILE = {}

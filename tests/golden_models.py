@@ -186,6 +186,18 @@ def build_model(fx):
     return getattr(M, fx.builder)(lin, dnn, **kw)
 
 
+def graph_signature(model):
+    """What identifies a built graph: inputs, layers (class + Keras-style name), weights (name + shape +
+    trainable) and the embedding planner's slots - plain lists, comparable with their JSON form."""
+    from deepctr_b200 import engine as E
+    layers = [[type(l).__name__, l.name] for l in model.layers if not isinstance(l, E.InputLayer)]
+    weights = [[w.name, list(w.shape), w.trainable] for w in model.weights]
+    slots = [[s.emb.name, s.input_name, s.maxlen, s.pool, s.mask_mode, s.len_name, s.weight_name, s.weight_mode,
+              s.dim, s.buf, s.col] for s in model.planner.slots]
+    return {"inputs": list(model.input_names), "layers": layers, "weights": weights, "slots": slots,
+            "fast": [model.planner.fast, getattr(model.planner, "fast_n", 0)]}
+
+
 def weight_map(fx, model):
     """{fixture key: deepctr_b200 Weight}; raises if the two weight sets differ (names or shapes)."""
     mine = {w.name: w for w in model.weights}

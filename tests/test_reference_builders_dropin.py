@@ -1,138 +1,44 @@
-"""CPU (build container only - needs /root/reference): "drop-in", literally.
+"""CPU: "drop-in", literally.
 
 The SOURCE FILES of the reference's five builders (deepctr/models/{deepfm,xdeepfm,dcn,autoint}.py,
-deepctr/models/sequence/din.py) are executed unmodified with their imports aliased to this package:
+deepctr/models/sequence/din.py), executed unmodified with their imports aliased to this package
+(tests/golden/generate_builders.py), built the graphs stored in tests/golden/reference_builders.json.
 
-    ..feature_column / ..inputs / ..layers.*      ->  deepctr_b200.feature_column / inputs / layers.*
-    tensorflow.keras.models.Model, .layers.{Dense,Flatten,Concatenate}  ->  deepctr_b200.engine
-
-The graphs they build must be the ones deepctr_b200.models builds for the same columns: same inputs,
-same layer sequence (class + Keras-style name), same weights (name + shape + trainable), same planner
-slots (i.e. the same single fused gather launch).  Graph construction needs no GPU.
+The graphs deepctr_b200.models builds for the same columns must be those: same inputs, same layer
+sequence (class + Keras-style name), same weights (name + shape + trainable), same planner slots (i.e.
+the same single fused gather launch).  Graph construction needs no GPU.
 """
-import importlib.util
+import inspect
+import json
 import os
-import sys
-import types
 
 import pytest
 
 import golden_models as G
 
-REF = "/root/reference/deepctr"
-pytestmark = pytest.mark.skipif(not os.path.isdir(REF), reason="reference tree not present (GPU box)")
-
-_FILES = {"DeepFM": ("models/deepfm.py", "models.deepfm"), "xDeepFM": ("models/xdeepfm.py", "models.xdeepfm"),
-          "DCN": ("models/dcn.py", "models.dcn"), "AutoInt": ("models/autoint.py", "models.autoint"),
-          "DIN": ("models/sequence/din.py", "models.sequence.din")}
-
-
-class _aliased(object):
-    """sys.modules entries that make the reference builder files import this package; restored on exit."""
-
-    def __enter__(self):
-        import deepctr_b200
-        from deepctr_b200 import engine, feature_column, inputs, layers
-        from deepctr_b200.layers import core, interaction, sequence, utils
-        self.saved = {k: v for k, v in sys.modules.items() if k == "tensorflow" or k.startswith("tensorflow.")
-                      or k == "refdrop" or k.startswith("refdrop.")}
-        for k in self.saved:
-            del sys.modules[k]
-
-        def mod(name, **attrs):
-            m = types.ModuleType(name)
-            m.__dict__.update(attrs)
-            m.__path__ = []
-            sys.modules[name] = m
-            return m
-        tf = mod("tensorflow")
-        tf.keras = mod("tensorflow.keras")
-        tf.keras.models = mod("tensorflow.keras.models", Model=engine.Model)
-        tf.keras.layers = mod("tensorflow.keras.layers", Dense=engine.Dense, Flatten=engine.Flatten,
-                              Concatenate=engine.Concatenate)
-        mod("refdrop")
-        mod("refdrop.models")
-        mod("refdrop.models.sequence")
-        sys.modules["refdrop.feature_column"] = feature_column
-        sys.modules["refdrop.inputs"] = inputs
-        sys.modules["refdrop.layers"] = layers
-        sys.modules["refdrop.layers.core"] = core
-        sys.modules["refdrop.layers.interaction"] = interaction
-        sys.modules["refdrop.layers.sequence"] = sequence
-        sys.modules["refdrop.layers.utils"] = utils
-        self.added = [k for k in sys.modules if k == "tensorflow" or k.startswith("tensorflow.")
-                      or k == "refdrop" or k.startswith("refdrop.")]
-        return self
-
-    def __exit__(self, *a):
-        for k in self.added:
-            sys.modules.pop(k, None)
-        sys.modules.update(self.saved)
-
-
-def _reference_builder(name):
-    rel, modname = _FILES[name]
-    full = "refdrop." + modname
-    spec = importlib.util.spec_from_file_location(full, os.path.join(REF, rel))
-    m = importlib.util.module_from_spec(spec)
-    sys.modules[full] = m
-    spec.loader.exec_module(m)            # the reference's unmodified source
-    return getattr(m, name)
-
-
-def _signature(model):
-    from deepctr_b200 import engine as E
-    layers = [(type(l).__name__, l.name) for l in model.layers if not isinstance(l, E.InputLayer)]
-    weights = [(w.name, tuple(w.shape), w.trainable) for w in model.weights]
-    slots = [(s.emb.name, s.input_name, s.maxlen, s.pool, s.mask_mode, s.len_name, s.weight_name, s.weight_mode,
-              s.dim, s.buf, s.col) for s in model.planner.slots]
-    return {"inputs": list(model.input_names), "layers": layers, "weights": weights, "slots": slots,
-            "fast": (model.planner.fast, getattr(model.planner, "fast_n", 0))}
-
-
-def _args(fx):
-    from deepctr_b200 import feature_column as FC
-    kw = dict(fx.kwargs)
-    for k in ("dnn_hidden_units", "cin_layer_size", "att_hidden_size", "fm_group"):
-        if k in kw:
-            kw[k] = tuple(kw[k])
-    lin, dnn = G.columns(fx, "linear", FC), G.columns(fx, "dnn", FC)
-    if fx.builder == "DIN":
-        return (dnn, ["item_id", "cate_id"]), kw
-    return (lin, dnn), kw
+with open(os.path.join(os.path.dirname(G.MODELS), "reference_builders.json")) as _f:
+    REF = json.load(_f)
+BUILDERS = ("DeepFM", "xDeepFM", "DCN", "AutoInt", "DIN")
 
 
 @pytest.mark.parametrize("name", G.CASES)
 def test_reference_builder_source_runs_on_this_package(name):
-    from deepctr_b200 import engine as E
-    from deepctr_b200 import models as M
     fx = G.Fixture(name)
-    args, kw = _args(fx)
-    with _aliased():
-        build = _reference_builder(fx.builder)
-        E.clear_session()
-        theirs = build(*args, **kw)
-    E.clear_session()
-    ours = getattr(M, fx.builder)(*args, **kw)
-    a, b = _signature(theirs), _signature(ours)
+    a = REF["graphs"][name]
+    b = json.loads(json.dumps(G.graph_signature(G.build_model(fx))))
     assert a["inputs"] == b["inputs"]
     assert a["weights"] == b["weights"]
     assert a["slots"] == b["slots"] and a["fast"] == b["fast"]
     # the op graph: same multiset of (layer class, name); the topological order may differ where the
     # reference builds a branch earlier than it consumes it
     assert sorted(a["layers"]) == sorted(b["layers"])
-    # and the reference-built graph carries the reference-produced weights by name
-    G.weight_map(fx, theirs)
 
 
 def test_reference_default_arguments_are_the_same():
     """every keyword and default of the five reference builders exists here with the same default."""
-    import inspect
     from deepctr_b200 import models as M
-    with _aliased():
-        for name in _FILES:
-            ref = inspect.signature(_reference_builder(name))
-            mine = inspect.signature(getattr(M, name))
-            assert list(ref.parameters) == list(mine.parameters), name
-            for k, p in ref.parameters.items():
-                assert p.default == mine.parameters[k].default, (name, k)
+    assert sorted(REF["defaults"]) == sorted(BUILDERS)
+    for name in BUILDERS:
+        mine = [[k, repr(p.default)] for k, p in inspect.signature(getattr(M, name)).parameters.items()]
+        assert [k for k, _ in REF["defaults"][name]] == [k for k, _ in mine], name
+        assert REF["defaults"][name] == mine, name
